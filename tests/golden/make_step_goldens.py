@@ -2,15 +2,17 @@
 
     python tests/golden/make_step_goldens.py synth180k     # BASELINE configs[1] geometry: synthetic KITTI-shape scan, 180 000 points,
                                                            # first step of the T=50 schedule   -> tests/golden/step_synth180k.npz
-    python tests/golden/make_step_goldens.py ply000123     # the reference's own fixture lidiff/Datasets/test/000123.ply preprocessed per
+    python tests/golden/make_step_goldens.py ply000123 <LiDiff checkout>/lidiff/Datasets/test/000123.ply
+                                                           # the reference's own fixture preprocessed per
                                                            # tools/diff_completion_pipeline.py:92-105, T=1 (timesteps [999]) + refinement
-                                                           #                                   -> tests/golden/step_000123.npz
+                                                           #       -> tests/golden/step_000123.npz, tests/golden/step_000123_refine.npz
 
 Everything is computed by the CPU oracle (fp32, `oracle/`) — about 2-4 minutes per case on 8 cores — so the tests only load the
-result.  To keep the fixtures small they hold: the 18 000 conditioning points (fp64), the calibrated BatchNorm tensors (the conv /
-linear weights are re-created from their seeds on the test machine and checked against a digest), digests of the noise tensors,
-per-level row counts + key checksums + pair counts (bit-exact quantities), and every 4th row of eps / x_next / refinement offsets
-plus fp64 sums over the full arrays.  /root/reference is read here only (for the .ply); the tests never touch it.
+result.  To keep the fixtures under 1 MB each they hold: the 18 000 conditioning points (for the synthetic scan their indices into
+range_filter(synthetic_scan(0)), for the .ply its float32 values), the calibrated BatchNorm tensors (the conv / linear weights are
+re-created from their seeds on the test machine and checked against a digest), digests of the noise tensors, per-level row counts
++ key checksums + pair counts (bit-exact quantities), every 8th row of eps / x_next, every 16th point of the refinement offsets
+(in a file of their own), plus fp64 sums over the full arrays.  The .ply is read here only; the tests never need it.
 """
 import hashlib
 import os
@@ -28,7 +30,8 @@ from oracle import me_cpu as ome                                     # noqa: E40
 from oracle.nets import random_state_dict                            # noqa: E402
 from oracle.pipeline import DiffCompletionOracle, farthest_point_sample    # noqa: E402
 
-STRIDE = 4
+STRIDE = 8
+REFINE_STRIDE = 16
 
 
 def digest(*tensors) -> str:
@@ -84,7 +87,7 @@ def level_stats(geom):
     return np.array(rows, np.int64), np.array(ksum, np.uint64), np.array(kxor, np.uint64), np.array(pairs, np.int64)
 
 
-def main(case):
+def main(case, ply=None):
     torch.set_num_threads(os.cpu_count() or 1)
     t0 = time.time()
     if case == "synth180k":
@@ -93,7 +96,7 @@ def main(case):
         T, refine = 50, False
     elif case == "ply000123":
         from lidiff_b200.synth import range_filter, read_ply_xyz
-        raw = range_filter(read_ply_xyz("/root/reference/lidiff/Datasets/test/000123.ply"))
+        raw = range_filter(read_ply_xyz(ply))
         T, refine = 1, True
     else:
         raise SystemExit(__doc__)
@@ -115,7 +118,10 @@ def main(case):
     hist = o.trace["hist"][0]
     eps, x_next = hist["eps"][0].float(), hist["x_next"][0].float()
     rows, ksum, kxor, pairs = level_stats(o.trace["geom"])
-    out = dict(part=part, stride=np.int64(STRIDE), weights_digest=np.array(wd), start_digest=np.array(digest(start)), step_digest=np.array(digest(step)),
+    # the synthetic scan is regenerated from its seed on the test machine: its indices are enough; the .ply holds float32 values
+    stored = dict(part_index=np.asarray(sel, np.int32)) if case == "synth180k" else dict(part=part.astype(np.float32))
+    assert case == "synth180k" or np.array_equal(stored["part"].astype(np.float64), part)
+    out = dict(**stored, stride=np.int64(STRIDE), weights_digest=np.array(wd), start_digest=np.array(digest(start)), step_digest=np.array(digest(step)),
                T=np.int64(T), level_rows=rows, level_key_sum=ksum, level_key_xor=kxor, pairs3=pairs,
                eps=eps[::STRIDE].numpy(), x_next=x_next[::STRIDE].numpy(),
                eps_sum=np.float64(eps.double().sum()), eps_abs_sum=np.float64(eps.double().abs().sum()),
@@ -129,6 +135,7 @@ def main(case):
     out["bn_keys"] = np.array(bn_keys)
     out["bn_sizes"] = np.array([v.size for v in bn_vals], np.int64)
     out["bn_vals"] = np.concatenate(bn_vals)
+    name = "000123" if case == "ply000123" else case
     if refine:
         post = o.postprocess_scan(completed, scan)
         off = o.refine.unet_refine(o.points_to_tensor(torch.from_numpy(post)[None, :, :])).reshape(-1, 6, 3)
@@ -137,14 +144,13 @@ def main(case):
         # refinement parity decoupled from the diffusion result: input = conditioning scan + 2 cm seeded noise
         rin = (scan + 0.02 * torch.randn(scan.shape, generator=torch.Generator().manual_seed(99), dtype=scan.dtype)).float()
         off2 = o.refine.unet_refine(o.points_to_tensor(rin)).reshape(-1, 6, 3)
-        out["refine_in_digest"] = np.array(digest(rin))
-        out["refine_stride"] = np.int64(4 * STRIDE)
-        out["refine_offsets"] = off2[::4 * STRIDE].numpy()
-        out["refine_offsets_abs_sum"] = np.float64(off2.double().abs().sum())
-    path = os.path.join(HERE, f"step_{'000123' if case == 'ply000123' else case}.npz")
+        np.savez_compressed(os.path.join(HERE, f"step_{name}_refine.npz"), refine_in_digest=np.array(digest(rin)),
+                            refine_stride=np.int64(REFINE_STRIDE), refine_offsets=off2[::REFINE_STRIDE].numpy(),
+                            refine_offsets_abs_sum=np.float64(off2.double().abs().sum()))
+    path = os.path.join(HERE, f"step_{name}.npz")
     np.savez_compressed(path, **out)
     print(f"wrote {path} ({os.path.getsize(path) / 1e6:.2f} MB); oracle step {t_step:.1f} s; rows {rows.tolist()} pairs {pairs.tolist()}; total {time.time() - t0:.0f} s")
 
 
 if __name__ == "__main__":
-    main(sys.argv[1] if len(sys.argv) > 1 else "")
+    main(sys.argv[1] if len(sys.argv) > 1 else "", sys.argv[2] if len(sys.argv) > 2 else None)

@@ -1,4 +1,6 @@
 """Import shims of SURVEY.md 8f-1: pytorch_lightning / natsort / open3d stand-ins the reference's inference script needs."""
+import importlib
+import json
 import os
 import sys
 
@@ -78,66 +80,67 @@ def test_open3d_fps_fails_loudly_without_gpu():
         pcd.farthest_point_down_sample(3)
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/lidiff/tools/diff_completion_pipeline.py"), reason="reference tree not mounted")
+REFERENCE = json.load(open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_on_shims.json")))
+
+
+def resolve(dotted):
+    """import the longest importable prefix of `dotted`, then walk the remaining attributes"""
+    parts = dotted.split(".")
+    for n in range(len(parts), 0, -1):
+        try:
+            obj = importlib.import_module(".".join(parts[:n]))
+        except ImportError:
+            continue
+        for a in parts[n:]:
+            obj = getattr(obj, a)
+        return obj
+    raise ImportError(dotted)
+
+
 def test_reference_pipeline_script_imports_on_the_shims():
-    """the reference's own inference script resolves every import against the shims and defines its classes unchanged"""
-    import importlib
-    sys.path.insert(0, "/root/reference")
-    try:
-        for m in [k for k in sys.modules if k == "lidiff" or k.startswith("lidiff.")]:
-            sys.modules.pop(m)
-        mod = importlib.import_module("lidiff.tools.diff_completion_pipeline")
-        from pytorch_lightning.core.lightning import LightningModule
-        assert issubclass(mod.DiffCompletion, LightningModule)
-        assert mod.o3d.__version__.endswith("lidiff_b200.shim") and callable(mod.natsorted)
-        assert mod.minknet.ME.__name__ == "MinkowskiEngine"
-    finally:
-        sys.path.remove("/root/reference")
-        for m in [k for k in sys.modules if k == "lidiff" or k.startswith("lidiff.")]:
-            sys.modules.pop(m)
+    """every name the reference's inference script (lidiff/tools/diff_completion_pipeline.py), its network module
+    (lidiff/models/minkunet.py) and its metrics module (lidiff/utils/metrics.py) take from a shimmed package resolves on the shims
+    (the names are recorded in tests/golden/reference_on_shims.json by tests/golden/make_reference_goldens.py)"""
+    names = REFERENCE["shim_names"]
+    assert set(names) == {"lidiff/tools/diff_completion_pipeline.py", "lidiff/models/minkunet.py", "lidiff/utils/metrics.py"}
+    for path, dotted in names.items():
+        for d in dotted:
+            assert resolve(d) is not None, f"{path}: {d}"
+    from pytorch_lightning.core.lightning import LightningModule
+    import MinkowskiEngine as ME
+    import natsort
+    import open3d as o3d
+    assert isinstance(LightningModule, type) and issubclass(LightningModule, torch.nn.Module)
+    assert issubclass(o3d.geometry.PointCloud, o3d.geometry.Geometry)
+    assert o3d.__version__.endswith("lidiff_b200.shim") and callable(natsort.natsorted)
+    assert ME.__name__ == "MinkowskiEngine"
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/lidiff/utils/metrics.py"), reason="reference tree not mounted")
 def test_reference_metrics_module_runs_on_the_open3d_shim():
-    """SURVEY 8f-4: /root/reference/lidiff/utils/metrics.py (RMSE, ChamferDistance, PrecisionRecall, CompletionIoU) unchanged on the
-    open3d shim; the nearest-neighbour distances it builds on are checked against scipy's exact k-d tree"""
-    import importlib
+    """SURVEY 8f-4: what the reference's lidiff/utils/metrics.py (RMSE, ChamferDistance, PrecisionRecall, CompletionIoU) computed on
+    the open3d shim (recorded in tests/golden/reference_on_shims.json) equals the same quantities from the shim's nearest-neighbour
+    distances, and those distances equal scipy's exact k-d tree"""
     from scipy.spatial import cKDTree
     import open3d as o3d
-    sys.path.insert(0, "/root/reference")
-    try:
-        for m in [k for k in sys.modules if k == "lidiff" or k.startswith("lidiff.")]:
-            sys.modules.pop(m)
-        metrics = importlib.import_module("lidiff.utils.metrics")
-        metrics.torch = torch                                     # the module uses `torch.Tensor` without importing torch
-        g = np.random.default_rng(3)
-        gt = g.normal(size=(6000, 3)) * [12, 12, 1.0]
-        pred = gt[g.choice(6000, 4000, replace=False)] + g.normal(size=(4000, 3)) * 0.05
-        pg, pp = o3d.geometry.PointCloud(gt), o3d.geometry.PointCloud(pred)
-        d_pg = np.asarray(pp.compute_point_cloud_distance(pg))
-        d_gp = np.asarray(pg.compute_point_cloud_distance(pp))
-        assert np.allclose(d_pg, cKDTree(gt).query(pred)[0], rtol=0, atol=1e-9) and np.allclose(d_gp, cKDTree(pred).query(gt)[0], rtol=0, atol=1e-9)
-        cd, rm = metrics.ChamferDistance(), metrics.RMSE()
-        cd.update(pg, pp); rm.update(pg, pp)
-        assert abs(cd.compute()[0] - 0.5 * (d_pg.mean() + d_gp.mean())) < 1e-12 and abs(rm.compute()[0] - d_pg.mean()) < 1e-12
-        pr = metrics.PrecisionRecall(0.05, 1.0, 20)
-        pr.update(pg, pp)
-        p, r, f1, t = pr.compute_at_threshold(0.1)
-        assert abs(p - 100.0 * (d_pg < t).mean()) < 1e-9 and abs(r - 100.0 * (d_gp < t).mean()) < 1e-9 and 0 < f1 <= 100
-        assert all(0 <= v <= 100.000001 for v in pr.compute_auc())            # percentages, normalised by the perfect predictor
-        iou = metrics.CompletionIoU(voxel_sizes=[2.0, 1.0, 0.5])       # (the default 0.1 m grid is a 1000^3 float64 histogram: 8 GB)
-        iou.update(pg, pp)
-        res = iou.compute()
-        assert set(res) == {2.0, 1.0, 0.5} and 0 < res[0.5] <= res[1.0] <= res[2.0] <= 1
-        assert not metrics.Metrics3D().prediction_is_empty(pp) and metrics.Metrics3D().prediction_is_empty(np.zeros((0, 3)))
-        assert metrics.Metrics3D.convert_to_pcd(pred).__class__ is o3d.geometry.PointCloud
-        # viewpoint mask of the training collation (collations.py:44-50): voxel-grid membership at 10 m
-        grid = o3d.geometry.VoxelGrid.create_from_point_cloud(pp, voxel_size=10.0)
-        inc = np.array(grid.check_if_included(o3d.utility.Vector3dVector(gt)))
-        org = pred.min(0) - 5.0
-        keys = {tuple(k) for k in np.floor((pred - org) / 10.0).astype(int)}
-        assert np.array_equal(inc, np.array([tuple(k) in keys for k in np.floor((gt - org) / 10.0).astype(int)]))
-    finally:
-        sys.path.remove("/root/reference")
-        for m in [k for k in sys.modules if k == "lidiff" or k.startswith("lidiff.")]:
-            sys.modules.pop(m)
+    ref = REFERENCE["metrics"]
+    g = np.random.default_rng(3)
+    gt = g.normal(size=(6000, 3)) * [12, 12, 1.0]
+    pred = gt[g.choice(6000, 4000, replace=False)] + g.normal(size=(4000, 3)) * 0.05
+    pg, pp = o3d.geometry.PointCloud(gt), o3d.geometry.PointCloud(pred)
+    d_pg = np.asarray(pp.compute_point_cloud_distance(pg))
+    d_gp = np.asarray(pg.compute_point_cloud_distance(pp))
+    assert np.allclose(d_pg, cKDTree(gt).query(pred)[0], rtol=0, atol=1e-9) and np.allclose(d_gp, cKDTree(pred).query(gt)[0], rtol=0, atol=1e-9)
+    assert abs(ref["chamfer"][0] - 0.5 * (d_pg.mean() + d_gp.mean())) < 1e-12 and abs(ref["rmse"][0] - d_pg.mean()) < 1e-12
+    p, r, f1, t = ref["precision_recall_at_0.1"]
+    assert abs(p - 100.0 * (d_pg < t).mean()) < 1e-9 and abs(r - 100.0 * (d_gp < t).mean()) < 1e-9 and 0 < f1 <= 100
+    assert all(0 <= v <= 100.000001 for v in ref["precision_recall_auc"])     # percentages, normalised by the perfect predictor
+    iou = {float(k): v for k, v in ref["completion_iou"].items()}             # (the default 0.1 m grid is a 1000^3 float64 histogram: 8 GB)
+    assert set(iou) == {2.0, 1.0, 0.5} and 0 < iou[0.5] <= iou[1.0] <= iou[2.0] <= 1
+    assert ref["prediction_is_empty"] == [False, True]
+    assert isinstance(pp, o3d.geometry.Geometry) and len(np.asarray(pp.points)) == 4000
+    # viewpoint mask of the training collation (collations.py:44-50): voxel-grid membership at 10 m
+    grid = o3d.geometry.VoxelGrid.create_from_point_cloud(pp, voxel_size=10.0)
+    inc = np.array(grid.check_if_included(o3d.utility.Vector3dVector(gt)))
+    org = pred.min(0) - 5.0
+    keys = {tuple(k) for k in np.floor((pred - org) / 10.0).astype(int)}
+    assert np.array_equal(inc, np.array([tuple(k) in keys for k in np.floor((gt - org) / 10.0).astype(int)]))
