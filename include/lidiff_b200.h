@@ -306,6 +306,39 @@ int lb2_guidance_dpm_step(void* h, void* stream, const float* eps_c, const float
 int lb2_farthest_point_sample(void* h, void* stream, const double* pts, int32_t n, int32_t n_samples,
                               int32_t* out_idx, double* dist_scratch);
 
+/* ---- evaluation metrics — lidiff/utils/metrics.py (RMSE, ChamferDistance, PrecisionRecall, CompletionIoU) and
+ * lidiff/utils/histogram_metrics.py (compute_hist_metrics), which use open3d's KDTreeFlann and dense np.histogramdd grids.
+ * Point clouds are fp64 (n, 3) row-major; n < 2^31.  Results stay on the device. */
+
+/* dist[i] = min_j |query[i] - ref[j]|, exact in fp64: squared distances are evaluated as (dx*dx + dy*dy) + dz*dz without FMA
+ * contraction and the square root is taken of the minimum, so dist equals numpy's np.sqrt(((q - r)**2).sum(1)) for the nearest r
+ * bit for bit.  A bounding-box hierarchy over the Morton-sorted reference keeps the cost ~log(nr) per query however far the query
+ * lies from the reference.  nq = 0 is a no-op; nr must be > 0.  scratch >= lb2_cloud_nn_scratch_bytes(nq, nr) (0 = bad sizes). */
+size_t lb2_cloud_nn_scratch_bytes(int64_t nq, int64_t nr);
+int lb2_cloud_nn_distance(void* h, void* stream, const double* query, int64_t nq, const double* ref, int64_t nr,
+                          void* scratch, double* dist);
+
+/* Two clouds on one voxel grid of bins^3 cells with per-axis edges `edges` (bins + 1 ascending fp64, np.linspace(-R, R, bins + 1)
+ * in the reference), binned like np.histogramdd: bin = searchsorted(edges, x, 'right') - 1, x == edges[bins] goes in the last bin,
+ * a point with a coordinate outside [edges[0], edges[bins]] is dropped.  The grid is never materialised (sorted bin keys).
+ *   n_a, n_b        points of a / b inside the grid;  occ_a, occ_b, occ_ab  occupied cells of a, of b, of both
+ *                   (CompletionIoU with a = ground truth: tp = occ_ab, fn = occ_a - tp, fp = occ_b - tp);
+ *   jsd_3d          scipy.spatial.distance.jensenshannon (base e) of the two count histograms;
+ *   jsd_bev         the same of the per-(x, y)-column numbers of occupied z cells (histogram_metrics.py with bev=True).
+ * Deterministic (fixed-order fp64 reductions).  bins < 2^21 (keys 2 * bins^3 fit 64 bits).
+ * scratch >= lb2_voxel_hist_scratch_bytes(na, nb); `out` is device memory. */
+typedef struct {
+    int64_t n_a, n_b;
+    int64_t occ_a, occ_b, occ_ab;
+    double  jsd_3d, jsd_bev;
+} lb2_voxel_hist_result;
+size_t lb2_voxel_hist_scratch_bytes(int64_t na, int64_t nb);
+int lb2_voxel_hist_compare(void* h, void* stream, const double* a, int64_t na, const double* b, int64_t nb,
+                           const double* edges, int32_t bins, void* scratch, lb2_voxel_hist_result* out);
+
+/* counts[t] = #{i : d[i] < thr[t]} (strict, as np.where(d < t)) for nthr <= 8192 ascending thresholds; counts int64[nthr]. */
+int lb2_threshold_counts(void* h, void* stream, const double* d, int64_t n, const double* thr, int32_t nthr, int64_t* counts);
+
 #ifdef __cplusplus
 }
 #endif

@@ -49,6 +49,11 @@ class ScatterDesc(C.Structure):
                 ("d_zero_rows", C.c_void_p), ("zero_rows_cap", C.c_int32)]
 
 
+class VoxelHistResult(C.Structure):
+    _fields_ = [("n_a", C.c_int64), ("n_b", C.c_int64), ("occ_a", C.c_int64), ("occ_b", C.c_int64), ("occ_ab", C.c_int64),
+                ("jsd_3d", C.c_double), ("jsd_bev", C.c_double)]
+
+
 class DpmCoef(C.Structure):
     _fields_ = [("c_sample", C.c_double), ("c_x0", C.c_double), ("c_noise", C.c_double),
                 ("sigma_s", C.c_double), ("alpha_s", C.c_double), ("inv_r0", C.c_double),
@@ -66,6 +71,8 @@ EXPORTS = [
     "lb2_nn_table_bytes", "lb2_nn_table_build", "lb2_nn_match_table",
     "lb2_nn_tree_bytes", "lb2_nn_tree_build", "lb2_nn_match_tree",
     "lb2_pair_list", "lb2_pair_list_scratch_bytes", "lb2_spconv_scatter", "lb2_spconv_scatter_supported",
+    "lb2_cloud_nn_scratch_bytes", "lb2_cloud_nn_distance", "lb2_voxel_hist_scratch_bytes", "lb2_voxel_hist_compare",
+    "lb2_threshold_counts",
 ]
 
 
@@ -133,6 +140,13 @@ class Lib:
         d.lb2_head_mlp.argtypes = [vp, vp, vp, i64, i64, vp, vp, vp, vp, i32, vp, i32, i32, i32, i32, i32, vp, i64, i64]
         d.lb2_guidance_dpm_step.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp, vp, i64, DpmCoef, vp, vp, vp, vp]
         d.lb2_farthest_point_sample.argtypes = [vp, vp, vp, i32, i32, vp, vp]
+        d.lb2_cloud_nn_scratch_bytes.argtypes = [i64, i64]
+        d.lb2_cloud_nn_scratch_bytes.restype = C.c_size_t
+        d.lb2_cloud_nn_distance.argtypes = [vp, vp, vp, i64, vp, i64, vp, vp]
+        d.lb2_voxel_hist_scratch_bytes.argtypes = [i64, i64]
+        d.lb2_voxel_hist_scratch_bytes.restype = C.c_size_t
+        d.lb2_voxel_hist_compare.argtypes = [vp, vp, vp, i64, vp, i64, vp, i32, vp, vp]
+        d.lb2_threshold_counts.argtypes = [vp, vp, vp, i64, vp, i32, vp]
         self._handles = {}
         self._lock = threading.Lock()
 
@@ -306,6 +320,26 @@ class Handle:
     def farthest_point_sample(self, pts, n, n_samples, out_idx, dist):
         self._check(self.dll.lb2_farthest_point_sample(self.hp, self._stream(), _ptr(pts), int(n), int(n_samples), _ptr(out_idx), _ptr(dist)),
                     "lb2_farthest_point_sample")
+
+    # -- evaluation metrics ----------------------------------------------------------------------------
+    def cloud_nn_scratch_bytes(self, nq, nr) -> int:
+        return int(self.dll.lb2_cloud_nn_scratch_bytes(int(nq), int(nr)))
+
+    def cloud_nn_distance(self, query, nq, ref, nr, scratch, dist):
+        self._check(self.dll.lb2_cloud_nn_distance(self.hp, self._stream(), _ptr(query), int(nq), _ptr(ref), int(nr), _ptr(scratch),
+                                                   _ptr(dist)), "lb2_cloud_nn_distance")
+
+    def voxel_hist_scratch_bytes(self, na, nb) -> int:
+        return int(self.dll.lb2_voxel_hist_scratch_bytes(int(na), int(nb)))
+
+    def voxel_hist_compare(self, a, na, b, nb, edges, bins, scratch, out):
+        """`out`: a device buffer of ctypes.sizeof(VoxelHistResult) bytes"""
+        self._check(self.dll.lb2_voxel_hist_compare(self.hp, self._stream(), _ptr(a), int(na), _ptr(b), int(nb), _ptr(edges), int(bins),
+                                                    _ptr(scratch), _ptr(out)), "lb2_voxel_hist_compare")
+
+    def threshold_counts(self, d, n, thr, nthr, counts):
+        self._check(self.dll.lb2_threshold_counts(self.hp, self._stream(), _ptr(d), int(n), _ptr(thr), int(nthr), _ptr(counts)),
+                    "lb2_threshold_counts")
 
 
 _LIB = None

@@ -90,3 +90,7 @@ __device__ __forceinline__ int floor_to_multiple(int v, int ts) {
     if ((v % ts != 0) && ((v < 0) != (ts < 0))) --q;
     return q * ts;
 }
+
+// Stable LSD radix sort of the low key_bits (<= 64) bits of n 64-bit keys into a permutation (coords.cu; used by metrics.cu).
+size_t lb2_sort_keys64_scratch_bytes(int n);
+int lb2_sort_keys64(Lb2Handle* h, cudaStream_t s, const unsigned long long* keys, int n, int key_bits, int* perm, void* scratch);

@@ -529,13 +529,15 @@ struct RsSrc {
                                  // mode 3: ro_key27(mask[vals_in[i]])   (first mask pass behind the Morton passes)
     const int4* coords;          // mode 2: ro_morton(coords[i])          (first Morton pass, value = i)
     const int* vals;             // values of the previous pass or NULL (value = i)
-    int mode, coord_shift;
+    const unsigned long long* keys64;   // mode 4: keys64[vals ? vals[i] : i] >> key_shift   (64-bit keys, lb2_sort_keys64)
+    int mode, coord_shift, key_shift;
 };
 __device__ __forceinline__ unsigned rs_key(const RsSrc& s, int i) {
     switch (s.mode) {
         case 0: return s.keys[i];
         case 1: return ro_key27(s.mask[i]);
         case 2: return ro_morton(s.coords[i], s.coord_shift);
+        case 4: return (unsigned)(s.keys64[s.vals ? s.vals[i] : i] >> s.key_shift);
         default: return ro_key27(s.mask[s.vals[i]]);
     }
 }
@@ -718,6 +720,36 @@ extern "C" int lb2_row_order(void* handle, void* stream, const uint32_t* row_mas
     LB2_POST_LAUNCH(h, "k_ro_scan");
     k_ro_scatter<<<cdiv(n_cap, 256), 256, 0, s>>>(row_mask, d_n, n_cap, kvol, bins, perm);
     LB2_POST_LAUNCH(h, "k_ro_scatter");
+    return LB2_OK;
+}
+
+// Stable LSD sort of 64-bit keys to a permutation (evaluation metrics, metrics.cu): perm[i] = index of the i-th smallest of the
+// low key_bits bits of keys[0..n).  Each pass reads its 9-bit digit of keys[previous permutation], so the keys are never moved.
+// scratch: [nblk][RS_BINS] histogram, [8][RS_BINS] per-pass totals, one int[n] ping-pong buffer.
+size_t lb2_sort_keys64_scratch_bytes(int n) {
+    return ((size_t)RS_BINS * (rs_blocks(n) + 8) + (size_t)n) * sizeof(int);
+}
+
+int lb2_sort_keys64(Lb2Handle* h, cudaStream_t s, const unsigned long long* keys, int n, int key_bits, int* perm, void* scratch) {
+    if (n <= 0) return LB2_OK;
+    const int nblk = rs_blocks(n);
+    const int npass = key_bits <= RS_BITS ? 1 : (key_bits + RS_BITS - 1) / RS_BITS;
+    int* hist = (int*)scratch;
+    int* total = hist + (size_t)RS_BINS * nblk;
+    int* tmp = total + 8 * RS_BINS;
+    if (cudaMemsetAsync(total, 0, (size_t)npass * RS_BINS * sizeof(int), s) != cudaSuccess) return lb2_fail(h, LB2_ERR_CUDA, "sort_keys64 memset%s", "");
+    const int* vin = nullptr;
+    for (int pass = 0; pass < npass; ++pass) {
+        int* vout = ((npass - 1 - pass) & 1) ? tmp : perm;                  // the last pass writes perm
+        RsSrc src;
+        src.keys = nullptr; src.mask = nullptr; src.coords = nullptr; src.vals = vin; src.keys64 = keys;
+        src.mode = 4; src.coord_shift = 0; src.key_shift = pass * RS_BITS;
+        k_rs_hist<<<nblk, 256, 0, s>>>(src, nullptr, n, 0, hist, total + pass * RS_BINS);
+        LB2_POST_LAUNCH(h, "k_rs_hist");
+        k_rs_scatter<<<nblk, 32 * RS_WARPS, 0, s>>>(src, nullptr, n, 0, hist, total + pass * RS_BINS, nullptr, vout);
+        LB2_POST_LAUNCH(h, "k_rs_scatter");
+        vin = vout;
+    }
     return LB2_OK;
 }
 

@@ -132,13 +132,17 @@ class PointCloud(Geometry):
 
     def compute_point_cloud_distance(self, target):
         """for every point of this cloud the Euclidean distance to its nearest point of `target` (open3d: KDTreeFlann 1-NN in
-        double precision) — what lidiff/utils/metrics.py builds RMSE / Chamfer distance / precision-recall on"""
+        double precision) — what lidiff/utils/metrics.py builds RMSE / Chamfer distance / precision-recall on.  On a GPU this is
+        lidiff_b200.metrics.nn_distance (exact fp64 bounding-box hierarchy search)."""
         import torch
         dev = "cuda" if torch.cuda.is_available() else "cpu"
         q64 = torch.as_tensor(np.asarray(self._points), dtype=torch.float64, device=dev)
         r64 = torch.as_tensor(np.asarray(target._points), dtype=torch.float64, device=dev)
         if q64.shape[0] == 0 or r64.shape[0] == 0:
             return np.zeros(q64.shape[0])
+        if dev == "cuda":
+            from lidiff_b200.metrics import nn_distance
+            return nn_distance(q64, r64).cpu().numpy()
         _, idx = _knn(q64.float(), r64.float(), 1)
         # the neighbour found in fp32 can differ from the fp64 one only between candidates equidistant to 1e-7: re-evaluate in fp64
         return (q64 - r64[idx[:, 0]]).norm(dim=1).cpu().numpy()
