@@ -129,6 +129,14 @@ int lb2_row_order(void* h, void* stream, const uint32_t* row_mask, const int32_t
 int lb2_tile_order(void* h, void* stream, const uint32_t* row_mask, const int32_t* row_perm, const int32_t* d_n, int32_t n_cap,
                    int32_t* order128, int32_t* order256, void* scratch);
 
+/* Dense / residual split of a map's row masks for the CTA-pair convolution (scheduling only: the pair set is unchanged).  For every
+ * 256-row super-tile of the row order `row_perm`, offset k is dense when at least min_rows of its rows have it (min_rows = 0: all offsets).
+ * dense_mask[row] = row_mask[row] & dense offsets of its super-tile, res_mask[row] = row_mask[row] & ~those (uint32[n_cap] each).
+ * The output-stationary kernel runs dense_mask (zero rows of sparse offsets are not multiplied); lb2_pair_list(row_mask = res_mask)
+ * compacts the rest for lb2_spconv_scatter. */
+int lb2_tile_split(void* h, void* stream, const uint32_t* row_mask, const int32_t* row_perm, const int32_t* d_n, int32_t n_cap,
+                   int32_t kvol, int32_t min_rows, uint32_t* dense_mask, uint32_t* res_mask);
+
 /* ---- sparse convolution  — replaces ME.MinkowskiConvolution(+Transpose) forward, with the
  * MinkowskiBatchNorm(eval)/MinkowskiReLU/residual-add/ME.cat/gate-multiply that follow it in
  * minkunet.py:13-80,431,464 fused as prologue/epilogue.
@@ -171,7 +179,8 @@ typedef struct {
     int32_t        mout_cap;
     const int32_t* row_perm;    /* execution order from lb2_row_order or NULL (natural order) */
     const uint32_t* row_mask;   /* per output row: bit k set <=> nbr[k][row] >= 0 (lb2_kernel_map's row_mask) or NULL.
-                                   A hint: lets the kernels skip the index loads of absent offsets */
+                                   Every variant (tensor-core and CUDA-core) convolves only the offsets whose bit is
+                                   set, so a subset (lb2_tile_split's dense_mask) convolves that subset of pairs */
     int32_t        npass;       /* 1 or 2 */
     lb2_conv_io    io[2];
     const int32_t* tile_order128;  /* from lb2_tile_order or NULL (tiles in row-order sequence, heaviest-looking last) */
@@ -189,7 +198,9 @@ int lb2_spconv_forward(void* h, void* stream, const lb2_conv_desc* d, int algo);
  * skipping one offset, e.g. the centre 13 of a 3^3 kernel), lb2_spconv_scatter computes
  *     out[pair_out] += in[pair_in] @ W[k]        (tensor cores, FP16x3, fp32 red.add; order-dependent last bits)
  * into a buffer that lb2_spconv_forward then consumes as `pre_add` while it handles the skipped offset with
- * kvol = 1.  Cout <= 128 and packed W[k] <= 96 KB (weight-stationary). */
+ * kvol = 1, or the dense offsets of lb2_tile_split.  Cout <= 256; W[k] stays in shared memory when it fits (Cout <= 128,
+ * Cin <= 256), otherwise it streams per 64-channel K chunk.
+ * lb2_pair_list's row_mask (optional): only the pairs (nbr[k][o], o) with bit k of row_mask[o] set. */
 typedef struct {
     int32_t        c1, c2, cout, kvol;
     const void*    weight_packed;
@@ -209,7 +220,7 @@ typedef struct {
 size_t lb2_pair_list_scratch_bytes(void);
 int lb2_pair_list(void* h, void* stream, const int32_t* nbr, int64_t nbr_stride, const int32_t* d_nout,
                   int32_t nout_cap, int32_t kvol, int32_t skip_k, int32_t* pair_in, int32_t* pair_out,
-                  int32_t* koff, int32_t* tile_off, void* scratch);
+                  int32_t* koff, int32_t* tile_off, void* scratch, const uint32_t* row_mask);
 int lb2_spconv_scatter_supported(int32_t c1, int32_t c2, int32_t cout, int32_t kvol);
 int lb2_spconv_scatter(void* h, void* stream, const lb2_scatter_desc* d);
 

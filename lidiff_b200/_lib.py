@@ -63,7 +63,7 @@ class DpmCoef(C.Structure):
 
 EXPORTS = [
     "lb2_create", "lb2_destroy", "lb2_last_error", "lb2_version", "lb2_launch_count", "lb2_read_status",
-    "lb2_set_option", "lb2_get_option", "lb2_tile_order",
+    "lb2_set_option", "lb2_get_option", "lb2_tile_order", "lb2_tile_split",
     "lb2_quantize", "lb2_unique_scratch_bytes", "lb2_unique_build", "lb2_voxel_mean", "lb2_kernel_map",
     "lb2_spconv_forward", "lb2_packed_weight_bytes", "lb2_pack_weights", "lb2_nn_match", "lb2_linear",
     "lb2_gate_mul", "lb2_gather_rows", "lb2_head_mlp", "lb2_kernel_map_self", "lb2_guidance_dpm_step", "lb2_farthest_point_sample",
@@ -116,12 +116,13 @@ class Lib:
         d.lb2_kernel_map_self.argtypes = [vp, vp, Grid, vp, vp, i32, i32, vp, i64, vp, vp]
         d.lb2_row_order.argtypes = [vp, vp, vp, vp, i32, i32, vp, vp, vp, i32]
         d.lb2_tile_order.argtypes = [vp, vp, vp, vp, vp, i32, vp, vp, vp]
+        d.lb2_tile_split.argtypes = [vp, vp, vp, vp, vp, i32, i32, i32, vp, vp]
         d.lb2_row_order_scratch_bytes.restype = C.c_size_t
         d.lb2_row_order_scratch_bytes.argtypes = [i32]
         d.lb2_spconv_forward.argtypes = [vp, vp, C.POINTER(ConvDesc), C.c_int]
         d.lb2_pack_weights.argtypes = [vp, vp, vp, i32, i32, i32, vp]
         d.lb2_nn_match.argtypes = [vp, vp, vp, vp, i32, vp, vp, i32, i32, vp]
-        d.lb2_pair_list.argtypes = [vp, vp, vp, i64, vp, i32, i32, i32, vp, vp, vp, vp, vp]
+        d.lb2_pair_list.argtypes = [vp, vp, vp, i64, vp, i32, i32, i32, vp, vp, vp, vp, vp, vp]
         d.lb2_pair_list_scratch_bytes.restype = C.c_size_t
         d.lb2_spconv_scatter.argtypes = [vp, vp, C.POINTER(ScatterDesc)]
         d.lb2_spconv_scatter_supported.argtypes = [i32, i32, i32, i32]
@@ -239,13 +240,17 @@ class Handle:
         self._check(self.dll.lb2_tile_order(self.hp, self._stream(), _ptr(row_mask), _ptr(row_perm), _ptr(d_n), int(n_cap), _ptr(order128),
                                             _ptr(order256), _ptr(scratch)), "lb2_tile_order")
 
+    def tile_split(self, row_mask, row_perm, d_n, n_cap, kvol, min_rows, dense_mask, res_mask):
+        self._check(self.dll.lb2_tile_split(self.hp, self._stream(), _ptr(row_mask), _ptr(row_perm), _ptr(d_n), int(n_cap), int(kvol), int(min_rows),
+                                            _ptr(dense_mask), _ptr(res_mask)), "lb2_tile_split")
+
     # -- conv ----------------------------------------------------------------------------------------
     def spconv(self, desc: ConvDesc, algo: int = ALGO_AUTO):
         self._check(self.dll.lb2_spconv_forward(self.hp, self._stream(), C.byref(desc), int(algo)), "lb2_spconv_forward")
 
-    def pair_list(self, nbr, nbr_stride, d_nout, nout_cap, kvol, skip_k, pair_in, pair_out, koff, tile_off, scratch):
+    def pair_list(self, nbr, nbr_stride, d_nout, nout_cap, kvol, skip_k, pair_in, pair_out, koff, tile_off, scratch, row_mask=None):
         self._check(self.dll.lb2_pair_list(self.hp, self._stream(), _ptr(nbr), int(nbr_stride), _ptr(d_nout), int(nout_cap), int(kvol), int(skip_k),
-                                           _ptr(pair_in), _ptr(pair_out), _ptr(koff), _ptr(tile_off), _ptr(scratch)), "lb2_pair_list")
+                                           _ptr(pair_in), _ptr(pair_out), _ptr(koff), _ptr(tile_off), _ptr(scratch), _ptr(row_mask)), "lb2_pair_list")
 
     def scatter_supported(self, c1, c2, cout, kvol) -> bool:
         return bool(self.dll.lb2_spconv_scatter_supported(int(c1), int(c2), int(cout), int(kvol)))

@@ -961,6 +961,33 @@ __global__ void __launch_bounds__(1024) k_tile_sort(const unsigned* __restrict__
     for (int u = nt256 + threadIdx.x; u < cap256; u += blockDim.x) order256[u] = -1;
 }
 
+// dense / residual split of the row masks per 256-row super-tile (the work item of k_spconv_tc_pair): an offset stays in the
+// output-stationary work when at least min_rows rows of the super-tile have it; otherwise the pairs of that offset go to the
+// residual mask, whose pairs lb2_pair_list compacts for the gather-GEMM-scatter kernel.  Every pair lands in exactly one of the two.
+__global__ void __launch_bounds__(256) k_tile_split(const unsigned* __restrict__ mask, const int* __restrict__ perm, const int* __restrict__ d_n,
+                                                    int n_cap, int kvol, int min_rows, unsigned* __restrict__ dense, unsigned* __restrict__ res) {
+    const int n = d_n ? min(*d_n, n_cap) : n_cap;
+    if (blockIdx.x * 256 >= n) return;                                 // uniform over the block
+    const int slot = blockIdx.x * 256 + threadIdx.x;
+    const int row = slot < n ? (perm ? __ldg(perm + slot) : slot) : -1;
+    const unsigned m = row >= 0 ? __ldg(mask + row) : 0u;
+    unsigned keep = 0;
+    for (int k = 0; k < kvol; ++k)
+        if (__syncthreads_count((m >> k) & 1u) >= min_rows) keep |= 1u << k;
+    if (row >= 0) { dense[row] = m & keep; res[row] = m & ~keep; }
+}
+
+extern "C" int lb2_tile_split(void* handle, void* stream, const uint32_t* row_mask, const int32_t* row_perm, const int32_t* d_n, int32_t n_cap,
+                              int32_t kvol, int32_t min_rows, uint32_t* dense_mask, uint32_t* res_mask) {
+    Lb2Handle* h = (Lb2Handle*)handle;
+    LB2_REQUIRE(h, h && row_mask && dense_mask && res_mask && n_cap > 0 && kvol >= 1 && kvol <= 32 && min_rows >= 0 && min_rows <= 256,
+                "tile_split");
+    cudaStream_t s = (cudaStream_t)stream;
+    k_tile_split<<<cdiv(n_cap, 256), 256, 0, s>>>(row_mask, row_perm, d_n, n_cap, kvol, min_rows, dense_mask, res_mask);
+    LB2_POST_LAUNCH(h, "k_tile_split");
+    return LB2_OK;
+}
+
 extern "C" int lb2_tile_order(void* handle, void* stream, const uint32_t* row_mask, const int32_t* row_perm, const int32_t* d_n, int32_t n_cap,
                               int32_t* order128, int32_t* order256, void* scratch) {
     Lb2Handle* h = (Lb2Handle*)handle;

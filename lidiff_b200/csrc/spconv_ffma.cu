@@ -29,12 +29,14 @@ struct FfmaParams {
     const int* d_mout;
     int mout_cap;
     const int* row_perm;
+    const unsigned* row_mask;   // offsets to convolve per output row (NULL: all of the map)
     lb2_conv_io io[2];
 };
 
 __global__ void __launch_bounds__(FF_THREADS) k_spconv_ffma(const FfmaParams p) {
     __shared__ int   idx_s[FF_BM];
     __shared__ int   row_s[FF_BM];
+    __shared__ unsigned mask_s[FF_BM];
     __shared__ float As[FF_BK][FF_BM + 4];
     __shared__ float Bs[FF_BK][FF_BN + 4];
 
@@ -57,13 +59,17 @@ __global__ void __launch_bounds__(FF_THREADS) k_spconv_ffma(const FfmaParams p) 
 #pragma unroll
         for (int j = 0; j < 4; ++j) acc[i][j] = 0.f;
 
-    if (t < FF_BM) row_s[t] = (m0 + t < M) ? (p.row_perm ? __ldg(p.row_perm + m0 + t) : m0 + t) : -1;
+    if (t < FF_BM) {
+        const int row = (m0 + t < M) ? (p.row_perm ? __ldg(p.row_perm + m0 + t) : m0 + t) : -1;
+        row_s[t] = row;
+        mask_s[t] = (row >= 0 && p.row_mask) ? __ldg(p.row_mask + row) : 0xffffffffu;
+    }
     __syncthreads();
     for (int k = 0; k < p.kvol; ++k) {
         int my = -1;
         if (t < FF_BM) {
             const int row = row_s[t];
-            if (row >= 0) my = p.nbr ? __ldg(p.nbr + (long long)k * p.nbr_stride + row) : row;
+            if (row >= 0 && ((mask_s[t] >> k) & 1u)) my = p.nbr ? __ldg(p.nbr + (long long)k * p.nbr_stride + row) : row;
             idx_s[t] = my;
         }
         if (!__syncthreads_or(my >= 0)) continue;      // nobody in this tile has a neighbour at offset k
@@ -173,7 +179,7 @@ int lb2_spconv_ffma_launch(Lb2Handle* h, cudaStream_t s, const lb2_conv_desc* d)
     FfmaParams p;
     p.c1 = d->c1; p.c2 = d->c2; p.cout = d->cout; p.kvol = d->kvol;
     p.W = d->weight; p.scale = d->scale; p.shift = d->shift; p.relu = d->relu;
-    p.nbr = d->nbr; p.nbr_stride = d->nbr_stride; p.d_mout = d->d_mout; p.mout_cap = d->mout_cap; p.row_perm = d->row_perm;
+    p.nbr = d->nbr; p.nbr_stride = d->nbr_stride; p.d_mout = d->d_mout; p.mout_cap = d->mout_cap; p.row_perm = d->row_perm; p.row_mask = d->row_mask;
     p.io[0] = d->io[0]; p.io[1] = d->io[d->npass > 1 ? 1 : 0];
     dim3 grid(cdiv(d->mout_cap, FF_BM), cdiv(d->cout, FF_BN), d->npass);
     k_spconv_ffma<<<grid, FF_THREADS, 0, s>>>(p);

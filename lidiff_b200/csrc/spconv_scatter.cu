@@ -9,7 +9,8 @@
 //
 // Persistent, weight-stationary: one CTA per SM walks a contiguous range of 128-pair tiles (sorted by k), so
 // the packed W[k] (all Cin chunks, <= 96 KB) is loaded into shared memory once per run of equal k and every
-// MMA reads B from there; only the gathered A rows stream through the stage ring.
+// MMA reads B from there; only the gathered A rows stream through the stage ring.  A W[k] that does not fit
+// (Cout 256: 256-384 KB) streams instead, one 64-column K chunk per slot of a two-slot ring, next to the A rows.
 //   warps 0-3 A producers (gather by pair_in, fp16 hi/lo split, SWIZZLE_128B image)     warp 4 MMA issuer
 //   warp 5 weight loader (cp.async.bulk)     warps 6-9 scatter epilogue (tcgen05.ld -> red.add), ping-pong TMEM
 // The scattered buffer is the `pre_add` input of the centre convolution, which applies BN/ReLU/residual/gate.
@@ -28,6 +29,7 @@ constexpr int MAX_STAGES = 4;
 constexpr int MAX_KVOL = 27;
 constexpr int SLAB_PITCH = 36;
 constexpr int SLAB_BYTES = BM * SLAB_PITCH * 4;
+constexpr int NBAR = 2 * MAX_STAGES + 8;
 
 struct Params {
     int c1, c2, cout, kvol, nchunks, stages, npass;
@@ -42,6 +44,7 @@ struct Params {
     const void* in2_h[2];
     float* out[2];
     int acc_stride, tmem_cols;
+    int stream_w;           // 1: W[k] streams through a 2-slot ring of K chunks instead of staying resident
 };
 
 __global__ void __launch_bounds__(THREADS, 1) k_spconv_scatter(const Params p) {
@@ -56,23 +59,24 @@ __global__ void __launch_bounds__(THREADS, 1) k_spconv_scatter(const Params p) {
     const uint32_t base = (raw + 1023u) & ~1023u;
     unsigned char* gen = smem_raw + (base - raw);
     const uint32_t b_tile = (uint32_t)p.cout * 128u;
-    const uint32_t w_bytes = (uint32_t)p.nchunks * 2u * b_tile;          // resident W[k]
+    const uint32_t w_bytes = (uint32_t)(p.stream_w ? 2 : p.nchunks) * 2u * b_tile;   // resident W[k] or the 2-slot chunk ring
     const uint32_t a_stage = 2u * A_TILE;
     unsigned char* a_gen = gen + w_bytes;
     const uint32_t a_base = base + w_bytes;
     float* slab = reinterpret_cast<float*>(a_gen + (size_t)p.stages * a_stage);         // [4 warps][32][SLAB_PITCH] epilogue transpose
     uint64_t* bars = reinterpret_cast<uint64_t*>(reinterpret_cast<unsigned char*>(slab) + SLAB_BYTES);
-    uint32_t* misc = reinterpret_cast<uint32_t*>(bars + 2 * MAX_STAGES + 6);
+    uint32_t* misc = reinterpret_cast<uint32_t*>(bars + NBAR);
     const uint32_t bar0 = smem_u32(bars);
     auto full_a = [&](int s) { return bar0 + 8u * s; };
     auto empty_a = [&](int s) { return bar0 + 8u * (MAX_STAGES + s); };
-    const uint32_t w_full = bar0 + 8u * (2 * MAX_STAGES), w_empty = bar0 + 8u * (2 * MAX_STAGES + 1);
-    auto acc_full = [&](int b) { return bar0 + 8u * (2 * MAX_STAGES + 2 + b); };
-    auto acc_empty = [&](int b) { return bar0 + 8u * (2 * MAX_STAGES + 4 + b); };
+    auto w_full = [&](int s) { return bar0 + 8u * (2 * MAX_STAGES + s); };          // slot 0 only when W[k] is resident
+    auto w_empty = [&](int s) { return bar0 + 8u * (2 * MAX_STAGES + 2 + s); };
+    auto acc_full = [&](int b) { return bar0 + 8u * (2 * MAX_STAGES + 4 + b); };
+    auto acc_empty = [&](int b) { return bar0 + 8u * (2 * MAX_STAGES + 6 + b); };
 
     if (threadIdx.x == 0) {
         for (int s = 0; s < p.stages; ++s) { mbar_init(full_a(s), 128); mbar_init(empty_a(s), 1); }
-        mbar_init(w_full, 1); mbar_init(w_empty, 1);
+        for (int s = 0; s < 2; ++s) { mbar_init(w_full(s), 1); mbar_init(w_empty(s), 1); }
         for (int b = 0; b < 2; ++b) { mbar_init(acc_full(b), 1); mbar_init(acc_empty(b), 128); }
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
@@ -149,9 +153,9 @@ __global__ void __launch_bounds__(THREADS, 1) k_spconv_scatter(const Params p) {
             for (int T = t_begin; T < t_end; ++T, ++j) {
                 int pass, k, pbase, cnt;
                 decode(T, pass, k, pbase, cnt);
-                if (k != cur_k || pass != cur_pass) {              // new run of equal k: its weights must have landed
+                if (!p.stream_w && (k != cur_k || pass != cur_pass)) {    // new run of equal k: its weights must have landed
                     ++wrun; cur_k = k; cur_pass = pass;
-                    mbar_wait(w_full, wrun & 1);
+                    mbar_wait(w_full(0), wrun & 1);
                     tc_fence_after();
                 }
                 const int buf = j & 1;
@@ -161,8 +165,9 @@ __global__ void __launch_bounds__(THREADS, 1) k_spconv_scatter(const Params p) {
                     const int s = it % p.stages;
                     mbar_wait(full_a(s), (it / p.stages) & 1);
                     tc_fence_after();
+                    if (p.stream_w) { mbar_wait(w_full(it & 1), (it >> 1) & 1); tc_fence_after(); }
                     const uint32_t a_hi = a_base + (uint32_t)s * a_stage, a_lo = a_hi + A_TILE;
-                    const uint32_t b_hi = base + (uint32_t)c * 2u * b_tile, b_lo = b_hi + b_tile;
+                    const uint32_t b_hi = base + (uint32_t)(p.stream_w ? (it & 1) : c) * 2u * b_tile, b_lo = b_hi + b_tile;
                     const int ksteps = min(KC, ctot - c * KC) >> 4;
                     for (int ks = 0; ks < ksteps; ++ks) {
                         const uint64_t dah = make_desc(a_hi + ks * 32), dal = make_desc(a_lo + ks * 32);
@@ -172,8 +177,10 @@ __global__ void __launch_bounds__(THREADS, 1) k_spconv_scatter(const Params p) {
                         umma(tmem_acc, dah, dbl, idesc, 1);
                     }
                     umma_commit(empty_a(s));
+                    if (p.stream_w) umma_commit(w_empty(it & 1));
                 }
                 umma_commit(acc_full(buf));
+                if (p.stream_w) continue;
                 // last tile of this run of equal k?  then the weights may be replaced once these MMAs are done
                 bool run_ends = (T + 1 == t_end);
                 if (!run_ends) {
@@ -181,23 +188,36 @@ __global__ void __launch_bounds__(THREADS, 1) k_spconv_scatter(const Params p) {
                     decode(T + 1, p2, k2, pb2, c2);
                     run_ends = (k2 != k) || (p2 != pass);
                 }
-                if (run_ends) umma_commit(w_empty);
+                if (run_ends) umma_commit(w_empty(0));
             }
         }
         __syncwarp();
     } else if (warp == 5) {
         // =========================== weight loader ===========================
-        if (lane == 0) {
+        if (lane == 0 && p.stream_w) {
+            int it = 0;
+            for (int T = t_begin; T < t_end; ++T) {
+                int pass, k, pbase, cnt;
+                decode(T, pass, k, pbase, cnt);
+                const unsigned char* src = p.wpacked + PACK_HEADER + (size_t)k * p.nchunks * 2u * b_tile;
+                for (int c = 0; c < p.nchunks; ++c, ++it) {
+                    const int s = it & 1;
+                    if (it >= 2) mbar_wait(w_empty(s), ((it >> 1) - 1) & 1);
+                    mbar_expect_tx(w_full(s), 2u * b_tile);
+                    bulk_g2s(base + (uint32_t)s * 2u * b_tile, src + (size_t)c * 2u * b_tile, 2u * b_tile, w_full(s));
+                }
+            }
+        } else if (lane == 0) {
             int wrun = -1, cur_k = -1, cur_pass = -1;
             for (int T = t_begin; T < t_end; ++T) {
                 int pass, k, pbase, cnt;
                 decode(T, pass, k, pbase, cnt);
                 if (k == cur_k && pass == cur_pass) continue;
                 ++wrun; cur_k = k; cur_pass = pass;
-                if (wrun >= 1) mbar_wait(w_empty, (wrun - 1) & 1);
+                if (wrun >= 1) mbar_wait(w_empty(0), (wrun - 1) & 1);
                 const unsigned char* src = p.wpacked + PACK_HEADER + (size_t)k * w_bytes;
-                mbar_expect_tx(w_full, w_bytes);
-                for (int c = 0; c < p.nchunks; ++c) bulk_g2s(base + (uint32_t)c * 2u * b_tile, src + (size_t)c * 2u * b_tile, 2u * b_tile, w_full);
+                mbar_expect_tx(w_full(0), w_bytes);
+                for (int c = 0; c < p.nchunks; ++c) bulk_g2s(base + (uint32_t)c * 2u * b_tile, src + (size_t)c * 2u * b_tile, 2u * b_tile, w_full(0));
             }
         }
         __syncwarp();
@@ -250,13 +270,14 @@ __global__ void __launch_bounds__(THREADS, 1) k_spconv_scatter(const Params p) {
 }
 
 // ---- pair lists of a kernel map, grouped by offset ------------------------------------------------------------------
+// row_mask (optional): only the pairs whose bit is set in their output row's mask (a subset of the map's pairs)
 __global__ void k_pair_count(const int* __restrict__ nbr, long long nbr_stride, const int* __restrict__ d_n, int n_cap, int skip_k,
-                             int* __restrict__ cnt) {
+                             const unsigned* __restrict__ row_mask, int* __restrict__ cnt) {
     const int k = blockIdx.y;
     if (k == skip_k) return;
     const int n = d_n ? min(*d_n, n_cap) : n_cap;
     const int o = blockIdx.x * blockDim.x + threadIdx.x;
-    const bool hit = o < n && nbr[(long long)k * nbr_stride + o] >= 0;
+    const bool hit = o < n && (!row_mask || ((row_mask[o] >> k) & 1u)) && nbr[(long long)k * nbr_stride + o] >= 0;   // as k_pair_fill
     const unsigned m = __ballot_sync(0xffffffffu, hit);
     if ((threadIdx.x & 31) == 0 && m) atomicAdd(cnt + k, __popc(m));
 }
@@ -270,12 +291,13 @@ __global__ void k_pair_scan(const int* __restrict__ cnt, int kvol, int* __restri
 }
 
 __global__ void k_pair_fill(const int* __restrict__ nbr, long long nbr_stride, const int* __restrict__ d_n, int n_cap, int skip_k,
-                            const int* __restrict__ koff, int* __restrict__ cursor, int* __restrict__ pair_in, int* __restrict__ pair_out) {
+                            const unsigned* __restrict__ row_mask, const int* __restrict__ koff, int* __restrict__ cursor,
+                            int* __restrict__ pair_in, int* __restrict__ pair_out) {
     const int k = blockIdx.y;
     if (k == skip_k) return;
     const int n = d_n ? min(*d_n, n_cap) : n_cap;
     const int o = blockIdx.x * blockDim.x + threadIdx.x;
-    const int v = o < n ? nbr[(long long)k * nbr_stride + o] : -1;
+    const int v = (o < n && (!row_mask || ((row_mask[o] >> k) & 1u))) ? nbr[(long long)k * nbr_stride + o] : -1;
     const unsigned m = __ballot_sync(0xffffffffu, v >= 0);
     if (!m) return;
     const int lane = threadIdx.x & 31;
@@ -295,17 +317,23 @@ __global__ void k_zero_rows(float* __restrict__ buf, const int* __restrict__ d_n
     if (t < (long long)n * c / 4) reinterpret_cast<float4*>(buf)[t] = make_float4(0.f, 0.f, 0.f, 0.f);
 }
 
-static size_t smem_bytes(int cin, int cout, int stages) {
-    const int nchunks = (cin + tc::KC - 1) / tc::KC;
-    return 1024 + (size_t)nchunks * 2 * cout * 128 + (size_t)stages * 2 * tc::A_TILE + SLAB_BYTES + (2 * MAX_STAGES + 6) * 8 + 64;
+constexpr size_t SMEM_LIMIT = 227 * 1024 - 256;        // 224 B of static smem
+
+// w_slots: K chunks of W[k] in shared memory (all of them: resident, 2: streamed)
+static size_t smem_bytes(int w_slots, int cout, int stages) {
+    return 1024 + (size_t)w_slots * 2 * cout * 128 + (size_t)stages * 2 * tc::A_TILE + SLAB_BYTES + NBAR * 8 + 64;
 }
+
+static int nchunks_of(int cin) { return (cin + tc::KC - 1) / tc::KC; }
+
+static bool stream_w(int cin, int cout) { return smem_bytes(nchunks_of(cin), cout, 2) > SMEM_LIMIT; }
 
 static bool shape_ok(int c1, int c2, int cout, int kvol) {
     const int ctot = c1 + c2;
     if (kvol < 1 || kvol > MAX_KVOL || ctot % 16 || ctot < 16) return false;
     if (c2 > 0 && (c1 % 8 || c2 % 8)) return false;
-    if (cout % 32 || cout < 32 || cout > 128) return false;
-    return smem_bytes(ctot, cout, 2) <= 227 * 1024 - 256;
+    if (cout % 32 || cout < 32 || cout > 256) return false;
+    return smem_bytes(stream_w(ctot, cout) ? 2 : nchunks_of(ctot), cout, 2) <= SMEM_LIMIT;
 }
 
 }  // namespace sc
@@ -314,7 +342,7 @@ extern "C" size_t lb2_pair_list_scratch_bytes(void) { return 2 * 32 * sizeof(int
 
 extern "C" int lb2_pair_list(void* handle, void* stream, const int32_t* nbr, int64_t nbr_stride, const int32_t* d_nout,
                              int32_t nout_cap, int32_t kvol, int32_t skip_k, int32_t* pair_in, int32_t* pair_out,
-                             int32_t* koff, int32_t* tile_off, void* scratch) {
+                             int32_t* koff, int32_t* tile_off, void* scratch, const uint32_t* row_mask) {
     Lb2Handle* h = (Lb2Handle*)handle;
     LB2_REQUIRE(h, h && nbr && pair_in && pair_out && koff && tile_off && scratch && nout_cap > 0 && kvol >= 1 && kvol <= sc::MAX_KVOL, "pair_list");
     cudaStream_t s = (cudaStream_t)stream;
@@ -322,11 +350,11 @@ extern "C" int lb2_pair_list(void* handle, void* stream, const int32_t* nbr, int
     int* cursor = cnt + 32;
     if (cudaMemsetAsync(cnt, 0, 64 * sizeof(int), s) != cudaSuccess) return lb2_fail(h, LB2_ERR_CUDA, "pair_list memset%s", "");
     dim3 grid(cdiv(nout_cap, 256), kvol);
-    sc::k_pair_count<<<grid, 256, 0, s>>>(nbr, nbr_stride, d_nout, nout_cap, skip_k, cnt);
+    sc::k_pair_count<<<grid, 256, 0, s>>>(nbr, nbr_stride, d_nout, nout_cap, skip_k, row_mask, cnt);
     LB2_POST_LAUNCH(h, "k_pair_count");
     sc::k_pair_scan<<<1, 32, 0, s>>>(cnt, kvol, koff, tile_off, cursor);
     LB2_POST_LAUNCH(h, "k_pair_scan");
-    sc::k_pair_fill<<<grid, 256, 0, s>>>(nbr, nbr_stride, d_nout, nout_cap, skip_k, koff, cursor, pair_in, pair_out);
+    sc::k_pair_fill<<<grid, 256, 0, s>>>(nbr, nbr_stride, d_nout, nout_cap, skip_k, row_mask, koff, cursor, pair_in, pair_out);
     LB2_POST_LAUNCH(h, "k_pair_fill");
     return LB2_OK;
 }
@@ -346,14 +374,18 @@ extern "C" int lb2_spconv_scatter(void* handle, void* stream, const lb2_scatter_
     p.pair_in = d->pair_in; p.pair_out = d->pair_out; p.koff = d->koff; p.tile_off = d->tile_off;
     for (int i = 0; i < 2; ++i) {
         const int j = d->npass > 1 ? i : 0;
-        LB2_REQUIRE(h, d->in1[j] && d->out[j] && ((d->c2 > 0) == (d->in2[j] != nullptr)), "spconv_scatter io");
+        const bool has_h = d->in1_h[j] && (d->c2 == 0 || d->in2_h[j]);        // the producers read the companions when all are given
+        const bool has_f = d->in1[j] && (d->c2 == 0 || d->in2[j]);
+        LB2_REQUIRE(h, (has_h || has_f) && d->out[j] && (d->c2 > 0 || (!d->in2[j] && !d->in2_h[j])), "spconv_scatter io");
         p.in1[i] = d->in1[j]; p.in2[i] = d->in2[j]; p.out[i] = d->out[j];
         p.in1_h[i] = d->in1_h[j]; p.in2_h[i] = d->in2_h[j];
     }
+    p.stream_w = sc::stream_w(d->c1 + d->c2, d->cout) ? 1 : 0;
+    const int w_slots = p.stream_w ? 2 : p.nchunks;
     int stages = sc::MAX_STAGES;
-    while (stages > 2 && sc::smem_bytes(d->c1 + d->c2, d->cout, stages) > 227 * 1024 - 256) --stages;
+    while (stages > 2 && sc::smem_bytes(w_slots, d->cout, stages) > sc::SMEM_LIMIT) --stages;
     p.stages = stages;
-    const int half = d->cout <= 32 ? 32 : d->cout <= 64 ? 64 : 128;
+    const int half = d->cout <= 32 ? 32 : d->cout <= 64 ? 64 : d->cout <= 128 ? 128 : 256;
     p.acc_stride = half; p.tmem_cols = 2 * half;
     if (d->zero_rows_cap > 0) {        // clear the rows the scatter adds into
         for (int i = 0; i < d->npass; ++i) {
@@ -362,10 +394,10 @@ extern "C" int lb2_spconv_scatter(void* handle, void* stream, const lb2_scatter_
         }
     }
     {
-        cudaError_t e = lb2_configure_smem(h, LB2_K_SCATTER, sc::k_spconv_scatter, (int)(227 * 1024 - 256));   // 224 B of static smem
+        cudaError_t e = lb2_configure_smem(h, LB2_K_SCATTER, sc::k_spconv_scatter, (int)sc::SMEM_LIMIT);
         if (e != cudaSuccess) return lb2_fail(h, LB2_ERR_CUDA, "k_spconv_scatter smem attribute: %s", cudaGetErrorString(e));
     }
-    sc::k_spconv_scatter<<<h->num_sms, sc::THREADS, sc::smem_bytes(d->c1 + d->c2, d->cout, stages), s>>>(p);
+    sc::k_spconv_scatter<<<h->num_sms, sc::THREADS, sc::smem_bytes(w_slots, d->cout, stages), s>>>(p);
     LB2_POST_LAUNCH(h, "k_spconv_scatter");
     return LB2_OK;
 }

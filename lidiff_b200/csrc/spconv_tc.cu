@@ -51,6 +51,7 @@ struct Params {
     const int* d_mout;
     int mout_cap;
     const int* row_perm;
+    const unsigned* row_mask;   // offsets to convolve per output row (NULL: all of the map)
     int stages, nchunks, tmem_cols, tot_col, group;     // tot_col: TMEM column of the running total; group: offsets per drain
     int nbuf, acc_stride;
     int ncta;                                           // output channels handled by one CTA (cout or cout/2): blockIdx.z picks the slice                               // ping-pong accumulators (2 when 3 regions fit in TMEM) and their column pitch
@@ -103,6 +104,7 @@ __global__ void __launch_bounds__(THREADS, 1) k_spconv_tc(const Params p) {
         const int slot = m0 + threadIdx.x;
         const int row = (slot < M) ? (p.row_perm ? __ldg(p.row_perm + slot) : slot) : -1;
         row_s[threadIdx.x] = row;
+        const uint32_t rmask = (row >= 0 && p.row_mask) ? __ldg(p.row_mask + row) : 0xffffffffu;
         uint32_t mymask = 0;
         for (int k0 = 0; k0 < p.kvol; k0 += 9) {        // 9 independent loads in flight, then the votes
             int v[9];
@@ -110,7 +112,7 @@ __global__ void __launch_bounds__(THREADS, 1) k_spconv_tc(const Params p) {
             for (int q = 0; q < 9; ++q) {
                 const int k = k0 + q;
                 v[q] = -1;
-                if (k < p.kvol && row >= 0) v[q] = p.nbr ? __ldg(p.nbr + (long long)k * p.nbr_stride + row) : row;
+                if (k < p.kvol && row >= 0 && ((rmask >> k) & 1u)) v[q] = p.nbr ? __ldg(p.nbr + (long long)k * p.nbr_stride + row) : row;
             }
 #pragma unroll
             for (int q = 0; q < 9; ++q) {
@@ -424,7 +426,7 @@ int lb2_spconv_tc_launch(Lb2Handle* h, cudaStream_t s, const lb2_conv_desc* d, b
     p.c1 = d->c1; p.c2 = d->c2; p.cout = d->cout; p.kvol = d->kvol;
     p.wpacked = (const unsigned char*)d->weight_packed;
     p.scale = d->scale; p.shift = d->shift; p.relu = d->relu;
-    p.nbr = d->nbr; p.nbr_stride = d->nbr_stride; p.d_mout = d->d_mout; p.mout_cap = d->mout_cap; p.row_perm = d->row_perm;
+    p.nbr = d->nbr; p.nbr_stride = d->nbr_stride; p.d_mout = d->d_mout; p.mout_cap = d->mout_cap; p.row_perm = d->row_perm; p.row_mask = d->row_mask;
     p.nchunks = (d->c1 + d->c2 + tc::KC - 1) / tc::KC;
     const int nsplit = (d->cout == 256 && h->opt[LB2_OPT_TC_NSPLIT]) ? 2 : 1;   // measured slower (A gathered twice): off by default     // 256 channels: two CTAs of 128 (drain overlap, 3 stages)
     p.ncta = d->cout / nsplit;

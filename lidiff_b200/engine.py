@@ -32,6 +32,9 @@ from .scheduler import DPMSolverMultistepScheduler
 
 GATE_NAMES = ("stage1", "stage2", "stage3", "stage4", "up1", "up2", "up3", "up4")
 GATE_LEVEL = (0, 1, 2, 3, 4, 3, 2, 1)
+# level -> tau of the dense / residual split of the Cout-256 convolutions (Geometry).  Measured on a B200 (bench.py, 180k points):
+# level 3 at tau 0.5 takes the Cout-256 class from 8.95 to 8.44 ms/step; level 4 (fewer sparse offsets per super-tile) is slower split
+SPLIT_TAU = {3: 0.5}
 BN_EPS = 1e-5
 
 
@@ -153,6 +156,19 @@ class Geometry:
         self.pair_out = [torch.zeros(26 * n_cap, **i32) if w else None for w in want]
         self.koff = [torch.zeros(28, **i32) for _ in range(self.pair_levels)]
         self.tile_off = [torch.zeros(28, **i32) for _ in range(self.pair_levels)]
+        # dense / residual split of the 3^3 maps of the dense levels for the Cout-256 convolutions (lb2_tile_split): per 256-row
+        # super-tile, the offsets that fewer than tau * 256 rows have leave the CTA-pair kernel and run as compacted pair lists
+        # through lb2_spconv_scatter.  LB2_SPLIT_TAU="3:0.5,4:0.5" (level:tau, tau = 0 = off) overrides SPLIT_TAU.
+        env = os.environ.get("LB2_SPLIT_TAU")
+        tau = dict(SPLIT_TAU) if env is None else {int(a): float(b) for a, b in (kv.split(":") for kv in env.split(",") if kv)}
+        ok = use_pairs and h.scatter_supported(256, 0, 256, 27)
+        self.split_min_rows = {l: math.ceil(t * 256) for l, t in tau.items() if ok and 0 < t and l < levels}
+        self.split_of = {}                                   # nbr pointer -> (dense mask, tile orders, pair_in, pair_out, koff, tile_off)
+        self.split_bufs = {l: (torch.zeros(n_cap, **i32), torch.zeros(n_cap, **i32),
+                               (torch.zeros((n_cap + 127) // 128, **i32), torch.zeros((n_cap + 255) // 256, **i32)),
+                               torch.zeros(27 * n_cap, **i32), torch.zeros(27 * n_cap, **i32), torch.zeros(28, **i32), torch.zeros(28, **i32),
+                               torch.zeros(64, **i32))      # pair-list counters: one set per level (levels build on different streams)
+                           for l in self.split_min_rows}
 
     def build(self, coords_f: torch.Tensor, n_points: int, after_levels=None, late_stream=None, late_done=None):
         """coords_f (n_points,4) fp32 integer-valued [b,x,y,z] -> all levels and maps (async).  `after_levels()` is called once the
@@ -193,6 +209,13 @@ class Geometry:
 
         def map3(l, **kw):
             one(self.grid[l], l, 3, 1 << l, self.nbr3[l], self.perm3[l], l, **kw)
+            if l in self.split_min_rows:
+                dense, res, to, p_in, p_out, koff, toff, scratch = self.split_bufs[l]
+                mask, perm = self.mask_of[self.nbr3[l].data_ptr()], self.perm3[l]
+                h.tile_split(mask, perm, self.d_n[l], N, 27, self.split_min_rows[l], dense, res)
+                h.tile_order(dense, perm, self.d_n[l], N, to[0], to[1], kw.get("to_scratch", self.to_scratch))
+                h.pair_list(self.nbr3[l], N, self.d_n[l], N, 27, -1, p_in, p_out, koff, toff, scratch, row_mask=res)
+                self.split_of[self.nbr3[l].data_ptr()] = (dense, to, p_in, p_out, koff, toff)
             if l < self.pair_levels and self.use_pairs and l in self.pair_level_set:
                 h.pair_list(self.nbr3[l], N, self.d_n[l], N, 27, 13, self.pair_in[l], self.pair_out[l], self.koff[l], self.tile_off[l], self.pl_scratch)
                 self.pairs_of[self.nbr3[l].data_ptr()] = l
@@ -428,7 +451,24 @@ class DenoiseEngine:
         pre = None
         geom_lvl = self._pairs_lookup.get(nbr.data_ptr()) if (nbr is not None and self.use_scatter and lay.Wpc is not None
                                                                and self.conv_algo != _lib.ALGO_FFMA) else None
-        if geom_lvl is not None:
+        split = None
+        if (geom_lvl is None and nbr is not None and lay.cout == 256 and lay.kvol == 27 and lay.Wp is not None
+                and self.conv_algo != _lib.ALGO_FFMA):
+            split = self.geom.split_of.get(nbr.data_ptr())
+        if split is not None:
+            # sparse offsets of each super-tile: out_split[pair_out] += in[pair_in] @ W[k], added by the pair kernel's epilogue
+            dense, to_dense, p_in, p_out, koff, toff = split
+            pre = self.buf(f"split.{lay.cout}", (2, cap, lay.cout))
+            sd = ScatterDesc()
+            sd.c1, sd.c2, sd.cout, sd.kvol = d.c1, d.c2, lay.cout, 27
+            sd.weight_packed = lay.Wp.data_ptr()
+            sd.pair_in, sd.pair_out, sd.koff, sd.tile_off = p_in.data_ptr(), p_out.data_ptr(), koff.data_ptr(), toff.data_ptr()
+            sd.npass = npass
+            for p in range(npass):
+                sd.in1[p], sd.in2[p], sd.out[p] = _ptr(f(in1), p), _ptr(f(in2), p), pre[p].data_ptr()
+                sd.in1_h[p], sd.in2_h[p] = _ptr(hh(in1), p), _ptr(hh(in2), p)
+            sd.d_zero_rows, sd.zero_rows_cap = d_m.data_ptr(), cap
+        elif geom_lvl is not None:
             # off-centre pairs: out_scatter[pair_out] += in[pair_in] @ W[k]; the centre runs below as a 1x1 conv with pre_add
             g, l = geom_lvl
             pre = self.buf(f"scatter.{lay.cout}", (2, cap, lay.cout))
@@ -445,14 +485,15 @@ class DenoiseEngine:
         else:
             sd = None
         map_ptr = nbr.data_ptr() if nbr is not None else None
-        d.cout, d.kvol = lay.cout, (1 if pre is not None else lay.kvol)
-        d.weight = (lay.Wc if pre is not None else lay.W).data_ptr()
-        wp = lay.Wpc if pre is not None else lay.Wp
+        centre = pre is not None and split is None
+        d.cout, d.kvol = lay.cout, (1 if centre else lay.kvol)
+        d.weight = (lay.Wc if centre else lay.W).data_ptr()
+        wp = lay.Wpc if centre else lay.Wp
         d.weight_packed = wp.data_ptr() if wp is not None else None
         d.scale = lay.scale.data_ptr() if lay.scale is not None else None
         d.shift = lay.shift.data_ptr() if lay.shift is not None else None
         d.relu = 1 if relu else 0
-        if pre is not None:
+        if centre:
             nbr = None                               # centre offset = identity map
         d.nbr = nbr.data_ptr() if nbr is not None else None
         d.nbr_stride = nbr.stride(0) if nbr is not None else cap
@@ -461,8 +502,12 @@ class DenoiseEngine:
         perm = self._perm_lookup.get(nbr.data_ptr()) if (nbr is not None and self.use_row_order) else None
         d.row_perm = perm.data_ptr() if perm is not None else None
         mask = self._mask_lookup.get(nbr.data_ptr()) if nbr is not None else None
+        if split is not None:
+            mask = split[0]
         d.row_mask = mask.data_ptr() if mask is not None else None
         to = self._tile_order_lookup.get(nbr.data_ptr()) if (nbr is not None and perm is not None) else None
+        if split is not None and to is not None:
+            to = split[1]
         d.tile_order128 = to[0].data_ptr() if to is not None else None
         d.tile_order256 = to[1].data_ptr() if to is not None else None
         res_h = hh(residual) if (residual is not None and residual.f is None) else None

@@ -31,6 +31,21 @@ def waste_report(geom, sizes):
         pairs = int(popc(m).sum())
         cur, lex, ident = issued(m[perm]), issued(np.sort(m)), issued(m)
         print(f"  waste L{l}: rows {n} pairs/row {pairs / n:.2f}; issued/pairs natural {ident / pairs:.2f} current {cur / pairs:.2f} mask-sorted {lex / pairs:.2f}")
+        if l < 2:
+            continue
+        # dense / residual split of the CTA-pair kernel's 256-row super-tiles (lb2_tile_split) for a few tau: issued dense slots x 256
+        # rows over pairs, and the compacted residual pairs over pairs (LB2_PROFILE_TAUS="0.25,0.5,0.75")
+        mp = m[perm]
+        mp = np.concatenate([mp, np.zeros((-n) % 256, np.uint32)]).reshape(-1, 256)
+        cnt = ((mp[:, :, None] >> np.arange(27, dtype=np.uint32)) & 1).sum(1)             # super-tiles x offsets: rows that have it
+        full = int(popc(np.bitwise_or.reduce(mp, axis=1)).sum()) * 256
+        row = [f"union {full / pairs:.2f}"]
+        for tau in [float(t) for t in os.environ.get("LB2_PROFILE_TAUS", "0.25,0.5,0.75").split(",")]:
+            keep = cnt >= int(np.ceil(tau * 256))
+            dense = int(keep.sum()) * 256
+            res = int((cnt * ~keep).sum())
+            row.append(f"tau {tau}: {dense / pairs:.2f} + {res / pairs:.2f}")
+        print(f"  split L{l} (issued dense slots / pairs + compacted pairs / pairs): " + "; ".join(row))
 
 
 def main():
